@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — mel-frames/sec through the CFM DiT estimator (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg1|cfg2|cfg3|cfg4] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg1|cfg2|cfg3|cfg4] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one complete ``CFMDecoder.forward`` ODE solve over one batch of synthetic inputs
 (SURVEY.md §8d): weights = reference-style init under manual_seed(0) with the adaLN gates re-drawn
@@ -15,6 +15,7 @@ N(0, 0.3²); inputs under manual_seed(1); z unmasked; CFG strength 3.
   cpu_baseline / --impl reference: the reference's own CPU path — the genuine modules staged under
            baseline/_ref (kind "reference"; oracle port if nothing is staged) — on host cores, bounded sample
   parity : utterances {first, second, middle, last} of the measured batch re-solved on the CPU (checker only)
+  --dump-outputs DIR: the mel the timed solve returned in its last step, as DIR/mel.npy (see dump_outputs)
 Multi-GPU (torchrun, one rank per GPU): weak scaling, the per-GPU batch is fixed, every rank owns its slice
 (value / e2e); the rank-0-owns-everything NCCL scatter/gather variant is timed beside it (root_scatter_gather,
 with the scatter+gather alone reported separately); at N = 8 BASELINE cfg4 as written (1024 = 128 per GPU)
@@ -23,6 +24,7 @@ rides along under the key "cfg4".
 from __future__ import annotations
 
 import argparse
+import atexit
 import ctypes as C
 import json
 import os
@@ -108,6 +110,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", f"--id={self.index}", f"--query-gpu={self.QUERY}",
                                           "--format=csv,noheader,nounits", "-lms", "200"],
                                          stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
+            atexit.register(self.proc.kill)         # a run that dies before stop() must not leave the sampler behind
         except Exception:
             self.proc = None
             return
@@ -422,7 +425,7 @@ def run_config(args, name, model, dev, rank, world, steps, warmup, flush, *, ful
     ms_dev, out_dev, per_dev = timed_checked(step_device, steps, "value")
     launches = (model.estimator.launch_count() - l0) // (2 if any(r["region"] == "value" for r in remeasured) else 1)
     res = {"name": name, "cfgd": cfgd, "Bglob": Bglob, "T": T, "frames": frames_global, "ms_dev": ms_dev, "per_dev": per_dev,
-           "out_dev": out_dev if (full and not bucketed) else None,
+           "out_dev": out_dev if (full and not bucketed) else None, "out_last": out_dev if args.dump_outputs else None,
            "launches": int(launches), "host_ms": host_ms, "n_warm": n_warm, "remeasured": remeasured, "inp": inp}
     if args.ncu_mode:
         return res
@@ -530,6 +533,23 @@ def run_vocoder(args, dev, mel, flush, steps=5):
     return out
 
 
+DUMP_BYTES = 60_000_000            # the .npy header and rounding stay well inside 64 MB
+
+
+def dump_outputs(out_dir, mel):
+    """Writes the (B, n_mel, T) mel the timed solve returned in its last step as out_dir/mel.npy in float32, so that
+    two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.  A batch
+    larger than DUMP_BYTES is cut to a fixed, seeded sample of utterances, kept in batch order."""
+    import numpy as np
+    mel = mel.detach().float().cpu()
+    if mel.numel() * 4 > DUMP_BYTES:
+        n = DUMP_BYTES // (mel[0].numel() * 4)
+        rows = torch.randperm(mel.shape[0], generator=torch.Generator().manual_seed(0))[:n].sort().values
+        mel = mel[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "mel.npy"), mel.numpy())
+
+
 def work_flops(cfgd, lens):
     nfe = cfgd["n_steps"] * NFE_PER_STEP[cfgd["method"]] * (2 if cfgd["cfg"] is not None else 1)
     lens = lens.double()
@@ -555,9 +575,15 @@ def main():
                          "convs, fp16 activations x fp16 hi/lo weights in 2 passes) or bf16x3 (3 passes everywhere); at N = 1 the OTHER mode "
                          "is measured beside it and reported under 'other_precision'")
     ap.add_argument("--no-second-precision", action="store_true", help="skip the secondary precision block")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps write the mel the last timed step returned "
+                                                          "(rank 0's batch slice) as DIR/mel.npy, float32, at most 64 MB")
     ap.add_argument("--ncu-mode", action="store_true",
                     help="for `ncu` launch lists only: honours --warmup < 3, skips e2e / instrumented / CPU legs (numbers printed under a profiler are never bench values)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed (--impl ours)")
     cfgd = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -582,14 +608,15 @@ def main():
     if rank == 0:
         sampler.start()                 # started BEFORE warm-up: nvidia-smi start-up stalls the driver for ~100 ms
     r = run_config(args, args.config, model, dev, rank, world, args.steps, args.warmup, flush, full=True, precision=args.precision)
+    clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r.pop("out_last"))
     if args.ncu_mode:
         if rank == 0:
-            sampler.stop()
             print(json.dumps({"ncu_mode": True, "ms_per_step_under_profiler": r["ms_dev"] / args.steps, "gpu_launches": r["launches"]}))
         if world > 1:
             dist.destroy_process_group()
         return
-    clocks = sampler.stop() if rank == 0 else None
     # the other precision mode on the same box, same inputs (decide-with-evidence block: throughput, parity, GEMM roofline)
     other = None
     if world == 1 and not args.no_second_precision and args.engine == "tcgen05":

@@ -7,11 +7,10 @@ baseline — never as the thing measured or shipped.  The product path
 (``stabletts_b200``) never imports this package and fails loudly when its CUDA
 library is missing.
 
-Parity pinning: the restatement in ``estimator_ref.py`` is checked (a) live
-against the reference's own importable ``models.estimator.Decoder`` whenever
-``/root/reference`` exists (authoring container), and (b) everywhere against
-the committed fixtures under ``tests/golden/`` which were produced by
-``oracle/make_golden.py`` from that same unmodified reference.  The ODE
+Parity pinning: the restatement in ``estimator_ref.py`` is checked against
+the committed fixtures under ``tests/golden/``, produced by
+``oracle/make_golden.py`` and ``oracle/make_golden_modules.py`` from the
+unmodified reference's own ``models.estimator.Decoder``.  The ODE
 stepping arithmetic belongs to the third-party ``torchdiffeq`` (unpinned in the
 reference's requirements.txt:14, absent here): fixed-grid tableaux are restated
 from the published algorithm — "parity unpinned" for solver behaviour.

@@ -8,8 +8,8 @@ same torch library calls as the reference (``F.conv1d``, dense-float-mask
 ``F.scaled_dot_product_attention``) so that, timed on host cores, it is a fair
 stand-in for the reference's own CPU path.
 
-Pinned by: ``tests/test_oracle.py`` (live against ``models.estimator.Decoder``
-when ``/root/reference`` exists; always against ``tests/golden/*.npz``).
+Pinned by: ``tests/test_oracle.py`` (against ``tests/golden/*.npz``, outputs of ``models.estimator.Decoder`` and its
+RoPE module).
 Solver stepping (``odeint_fixed``) restates torchdiffeq's fixed-grid tableaux
 from the published algorithm: parity unpinned for solver behaviour.
 """

@@ -1,8 +1,6 @@
-"""Pins the oracle: restatement vs the committed reference-generated fixtures (always) and vs
-the live reference modules (only where /root/reference exists).  CPU only."""
+"""Pins the oracle: restatement vs the committed fixtures generated from the reference's own modules.  CPU only."""
+import json
 import os
-import sys
-import types
 
 import numpy as np
 import pytest
@@ -64,26 +62,22 @@ def test_solve_vs_golden(name, golden_dir):
     assert e_max < 1e-4 and e_l2 < 1e-4, (e_max, e_l2)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference checkout only exists in the authoring container")
-def test_live_reference_modules():
-    sys.path.insert(0, "/root/reference")
-    if "torchdiffeq" not in sys.modules:
-        stub = types.ModuleType("torchdiffeq")
-        stub.odeint = lambda f, y0, t, method=None, rtol=None, atol=None: R.odeint_fixed(f, y0, t, method)[None]
-        sys.modules["torchdiffeq"] = stub
-    from models.estimator import Decoder
-    from models.diffusion_transformer import RotaryPositionalEmbeddings
-    dec = Decoder(80, 80, 256, 80, 1024, 0.1, 6, 4, 3, 256).eval()
+def test_live_reference_modules(golden_dir):
+    """The restatement against the reference's Decoder and RotaryPositionalEmbeddings called on the same weights and
+    inputs (oracle/make_golden_modules.py records their outputs)."""
+    from oracle.make_golden_modules import DECODER_CALL as cs, ROPE_DIMS, rope_query
+    g = np.load(os.path.join(golden_dir, "decoder_rope.npz"))
     st = state_for(80)
-    dec.load_state_dict(st, strict=True)
-    inp = weights.make_inputs(99, [70, 45], 70, 80, t_per_sample=True)
+    with open(os.path.join(golden_dir, "reference_state_dicts.json")) as f:        # what load_state_dict(strict=True) checks
+        assert [[k, list(v.shape)] for k, v in st.items()] == json.load(f)["Decoder"]
+    inp = weights.make_inputs(cs["seed"], cs["lengths"], cs["T"], 80, t_per_sample=cs["t_per_sample"])
     with torch.inference_mode():
-        ref = dec(inp["t"], inp["x"], inp["mask"], inp["mu"], inp["c"])
         out = R.estimator_forward(st, inp["t"], inp["x"], inp["mask"], inp["mu"], inp["c"])
-    assert rel_errs(out, ref)[0] < TOL
+    assert rel_errs(out, torch.from_numpy(g["decoder_out"]))[0] < TOL
     # RoPE restatement is bit-exact against the module (SURVEY.md §8a a10)
-    q = torch.randn(2, 4, 37, 64)
-    assert torch.equal(R.rope_partial(q, 32), RotaryPositionalEmbeddings(32)(q))
+    q = rope_query()
+    assert abs(weights.checksum([q]) - float(g["rope_q_checksum"])) < 1e-6 * abs(float(g["rope_q_checksum"])), "RNG drift"
+    assert torch.equal(R.rope_partial(q, ROPE_DIMS), torch.from_numpy(g["rope_out"]))
 
 
 def test_padding_is_not_inert():

@@ -1,5 +1,6 @@
 """Row f2 (SURVEY.md §8f): TextEncoder on the estimator's kernels.  CPU: oracle vs reference-generated
-fixtures and the live module; state_dict inventory of the drop-in.  GPU: CUDA path vs fixtures (1e-3)."""
+fixtures; state_dict inventory of the drop-in vs the reference module's.  GPU: CUDA path vs fixtures (1e-3)."""
+import json
 import os
 
 import numpy as np
@@ -22,18 +23,15 @@ def test_oracle_vs_golden(name, golden_dir):
     assert torch.equal(m, torch.from_numpy(g["mask"]))
 
 
-def test_drop_in_inventory():
+def test_drop_in_inventory(golden_dir):
     import __graft_entry__ as ge
     ge.build()
     from stabletts_b200 import TextEncoder
     m = TextEncoder(401, 80, 256, 1024, 4, 3, 3, 0.1, 256)
     assert list(m.state_dict().keys()) == list(T.param_shapes().keys())
     m.load_state_dict(T.make_state(3), strict=True)
-    if os.path.isdir("/root/reference"):
-        import sys
-        sys.path.insert(0, "/root/reference")
-        from models.text_encoder import TextEncoder as Ref
-        assert list(Ref(401, 80, 256, 1024, 4, 3, 3, 0.1, 256).state_dict().keys()) == list(m.state_dict().keys())
+    with open(os.path.join(golden_dir, "reference_state_dicts.json")) as f:       # the reference's TextEncoder, same sizes
+        assert [[k, list(v.shape)] for k, v in m.state_dict().items()] == json.load(f)["TextEncoder"]
     ids, c, lens = T.make_inputs(1, [4], 4)
     with pytest.raises(NotImplementedError):                   # train() mode + autograd: no silent detached output
         m(ids, c, lens)

@@ -1,10 +1,9 @@
 """Row f4 (SURVEY.md §8f): the vocoder hand-off.  CPU: state_dict inventory of the drop-in against the oracle's restated
-inventory and (where /root/reference exists) the unmodified reference Vocos.  GPU: the CUDA path through the C ABI against
+inventory and the unmodified reference Vocos's (as recorded in tests/golden).  GPU: the CUDA path through the C ABI against
 the fixtures generated from the unmodified reference (tests/golden/vocos_*.npz, 1e-3) and against the oracle at sizes that
 reach the 2-CTA GEMM kernel; size-independent properties (batch independence, frame-count scaling of the output)."""
+import json
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -14,7 +13,7 @@ from conftest import rel_errs
 from oracle import vocoder_ref as V
 
 
-def test_drop_in_inventory_matches_reference_keys():
+def test_drop_in_inventory_matches_reference_keys(golden_dir):
     import __graft_entry__ as ge
     ge.build()
     from stabletts_b200 import Vocos
@@ -23,12 +22,8 @@ def test_drop_in_inventory_matches_reference_keys():
     got = {k: tuple(v.shape) for k, v in m.state_dict().items()}
     assert list(got) == list(want) and got == dict(want)
     m.load_state_dict(V.make_state(), strict=True)
-    if os.path.isdir("/root/reference/vocoders/vocos"):          # the vocoder's `models` package shadows the TTS one: own process
-        code = ("import sys; sys.path.insert(0, '/root/reference/vocoders/vocos');"
-                "from config import MelConfig, VocosConfig; from models.model import Vocos;"
-                "print('\\n'.join(Vocos(VocosConfig(), MelConfig()).state_dict().keys()))")
-        ref_keys = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, check=True).stdout.split()
-        assert ref_keys == list(got)
+    with open(os.path.join(golden_dir, "reference_state_dicts.json")) as f:     # Vocos(VocosConfig(), MelConfig())
+        assert [(k, tuple(v)) for k, v in json.load(f)["Vocos"]] == list(got.items())
     with pytest.raises(RuntimeError, match="CUDA"):
         m.eval()(torch.zeros(1, 128, 4))
 
